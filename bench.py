@@ -2,6 +2,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (sm_100a kernels)
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU path (oracle port)
+  ... --dump-outputs DIR                                    also write the pred_ids of the last timed step(s) to DIR/*.npy
 
 One "step" = one PREDICT pass of model.bert_bilstm_crf.build_graph over one synthetic
 MSRA-shaped batch (BERT-base encoder -> BiLSTM -> logits -> CRF log-likelihood + Viterbi),
@@ -29,6 +30,14 @@ METRIC = "sentences/sec bert_bilstm_crf MSRA L=128"
 WORKLOAD = ("bert_bilstm_crf msra seq_len=128 bs=64/GPU PREDICT step: BERT-base fwd (12L, H768) + BiLSTM(H128, relu) "
             "+ logits + CRF Viterbi -> pred_ids (the log-likelihood is part of the graph but PREDICT does not fetch it, as "
             "in the reference's Estimator); bf16 tcgen05 GEMM operands, fp32 residual/LSTM/CRF; MSRA-shaped lengths")
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, as float32 (the tags are small integers, exact in float32), so that
+    two builds run with the same arguments can be compared output for output."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def measured_peaks():
@@ -275,10 +284,12 @@ def run_reference(args):
         feats = synthetic.msra_batch(n_sent, SEQ_LEN, seed=1000 + i)
         t0 = time.perf_counter()
         with torch.no_grad():
-            omodels.bert_bilstm_crf(w, feats, params, dtype=torch.float32)
+            out = omodels.bert_bilstm_crf(w, feats, params, dtype=torch.float32)
         dt = time.perf_counter() - t0
         if i >= args.warmup:
             per_step.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pred_ids": np.asarray(out["pred_ids"])})
     total = float(sum(per_step))
     value = n_sent * len(per_step) / total
     line = {
@@ -532,10 +543,13 @@ def run_ours(args):
         flush.zero_()
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        step_resident(i)
+        last_pred = step_resident(i)
         e.record()
         evs.append((s, e))
     barrier()
+    # --dump-outputs: this loop's last step, and below the last batch of every timed pipeline configuration (each one, not
+    # only the one that sets `value`: that choice is made by timing, the set of configurations by the arguments)
+    outputs = {"pred_ids": last_pred.cpu().numpy()}
     launches = _lib.LAUNCHES - l0
     t_res = sum(s.elapsed_time(e) for s, e in evs) / 1e3
 
@@ -567,7 +581,7 @@ def run_ours(args):
             def run(j, nbat):
                 grp = groups if nbat == G else dev_group(nbat)      # the last call of the K steps may hold fewer batches
                 with torch.cuda.stream(side[j % NS]):
-                    est.predict_device(grp[j % len(grp)])
+                    return est.predict_device(grp[j % len(grp)])
             for j in range(2 * NS):
                 run(j, G)
             barrier()
@@ -576,21 +590,21 @@ def run_ours(args):
             for st in side:
                 st.wait_event(s)
             for j, nbat in calls:
-                run(j, nbat)
+                last_pred = run(j, nbat)
             for st in side:
                 torch.cuda.current_stream().wait_stream(st)
             e.record()
             barrier()
         finally:
             _ops.DEFAULT_TILE = 0
-        return s.elapsed_time(e) / 1e3
+        return s.elapsed_time(e) / 1e3, last_pred[-B_PER_GPU:].cpu().numpy()     # the last call's last 64-sentence batch
 
     combos = [(max(2, args.streams), 1), (max(1, args.group_streams), max(1, args.group))]
     if args.sweep:
         combos = sorted(set(combos + [(1, 2), (2, 2), (3, 2), (1, 4), (2, 4), (3, 4), (4, 4), (2, 6), (2, 8), (3, 8), (2, 1), (3, 1)]))
     pipe = {}
     for NS_, G_ in combos:
-        t = time_pipeline(NS_, G_)
+        t, outputs[f"pred_ids_pipeline_streams{NS_}_batches{G_}"] = time_pipeline(NS_, G_)
         if dist is not None:                        # max over ranks decides, every rank must pick the same combination
             tt = torch.tensor([t], device="cuda", dtype=torch.float64)
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -815,6 +829,8 @@ def run_ours(args):
             line["cpu_baseline"] = cpu
         line.update(extra)
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -833,7 +849,12 @@ def main():
     ap.add_argument("--group", type=int, default=4, help="batches stacked per PREDICT call in the second pipeline configuration")
     ap.add_argument("--group-streams", dest="group_streams", type=int, default=2, help="CUDA streams of the stacked configuration")
     ap.add_argument("--sweep", action="store_true", help="time more (streams, batches per call) combinations")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the pred_ids [64, 128] of the last timed step (rank 0) to DIR/pred_ids.npy, "
+                         "and those of the last batch of each timed pipeline configuration to DIR/pred_ids_pipeline_*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,6 +6,10 @@ Outputs (committed):
                               tokens (pins crf_decode's zero-fill), entity micro / weighted F1 by
                               chinesener_b200.evaluation (pins the evaluator against BASELINE.md §2)
   msra_bert_bilstm_crf_sample.pkl   first 48 sentences of data/msra/bert_bilstm_crf_predict.pkl
+
+`python tests/golden/make_golden.py --sample-reports` needs only the committed sample and scikit-learn:
+  msra_bert_bilstm_crf_sample_reports.json   the sample's tag-level report by scikit-learn (the library the reference's
+                              evaluation.py:38-46 uses for it) and its entity-level counts and F1
 """
 import glob
 import json
@@ -49,5 +53,27 @@ def main():
     pickle.dump(sample, open(os.path.join(out, "msra_bert_bilstm_crf_sample.pkl"), "wb"))
 
 
+def sample_reports():
+    from sklearn.metrics import precision_recall_fscore_support
+    from chinesener_b200.tools.predict_utils import process_prediction
+    out = os.path.join(ROOT, "tests", "golden")
+    idx2tag = {int(k): v for k, v in json.load(open(os.path.join(out, "predict_pickle_stats.json")))["idx2tag_msra"].items()}
+    sample = [process_prediction(dict(s), idx2tag) for s in pickle.load(open(os.path.join(out, "msra_bert_bilstm_crf_sample.pkl"), "rb"))]
+    y_true = [int(t) for s in sample for t in s["label_ids"]]
+    y_pred = [int(t) for s in sample for t in s["pred_ids"]]
+    labels = [k for k, v in sorted(idx2tag.items()) if v not in ("[PAD]", "[CLS]", "[SEP]")]
+    p, r, f, n = precision_recall_fscore_support(y_true, y_pred, labels=labels, average=None, zero_division=0)
+    wp, wr, wf, _ = precision_recall_fscore_support(y_true, y_pred, labels=labels, average="weighted", zero_division=0)
+    tag = {str(lab): {"precision": float(p[i]), "recall": float(r[i]), "f1-score": float(f[i]), "support": int(n[i])}
+           for i, lab in enumerate(labels)}
+    tag["weighted avg"] = {"precision": float(wp), "recall": float(wr), "f1-score": float(wf)}
+    ent = evaluation.entity_report([s["labels"] for s in sample], [s["preds"] for s in sample])
+    json.dump({"n_tokens": len(y_true), "tag_report_sklearn": tag, "entity_report": ent},
+              open(os.path.join(out, "msra_bert_bilstm_crf_sample_reports.json"), "w"), indent=1)
+
+
 if __name__ == "__main__":
-    main()
+    if "--sample-reports" in sys.argv:
+        sample_reports()
+    else:
+        main()

@@ -1,12 +1,10 @@
 """Golden for the dataset preparation path (SURVEY 8(f) rank 1): the first 24 sentences of the reference's MSRA test split
 (raw `sentences.txt` / `tags.txt` lines — data, ~4 KB) with the featurisation the REFERENCE produced for them, read back
 from its shipped prediction pickle `data/msra/bilstm_crf_predict.pkl` (tokens, label_ids under the giga tokenizer,
-max_seq_len 150), plus `data/msra/data_params.pkl` (n_sample / max_seq_len / label_size / tag2idx) and whole-split digests
-of the tokens and label_ids of all 3442 test sentences.  Needs /root/reference:
+max_seq_len 150), plus `data/msra/data_params.pkl` (n_sample / max_seq_len / label_size / tag2idx).  Needs /root/reference:
 
     python tests/golden/make_msra_sample_golden.py
 """
-import hashlib
 import json
 import os
 import pickle
@@ -14,20 +12,6 @@ import pickle
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF = "/root/reference/data/msra"
 N = 24
-
-
-def digest_tokens(rows):
-    h = hashlib.sha256()
-    for row in rows:
-        h.update("\x1f".join(row).encode("utf-8") + b"\n")
-    return h.hexdigest()
-
-
-def digest_ids(rows):
-    h = hashlib.sha256()
-    for row in rows:
-        h.update(bytes(int(x) for x in row))
-    return h.hexdigest()
 
 
 if __name__ == "__main__":
@@ -42,8 +26,7 @@ if __name__ == "__main__":
         "sentences": sent[:N], "tags": tags[:N], "tokens": toks[:N], "label_ids": labs[:N],
         "giga_vocab_subset": vocab,               # enough of the giga vocabulary to tokenise the sample
         "data_params": {k: (v if not isinstance(v, dict) else {str(a): b for a, b in v.items()}) for k, v in dp.items()},
-        "n_test": len(pred), "tokens_sha256": digest_tokens(toks), "label_ids_sha256": digest_ids(labs),
     }
     with open(os.path.join(HERE, "msra_sample.json"), "w", encoding="utf-8") as f:
         json.dump(out, f, ensure_ascii=False, indent=0)
-    print(len(pred), out["tokens_sha256"][:12], out["label_ids_sha256"][:12], os.path.getsize(os.path.join(HERE, "msra_sample.json")))
+    print(len(pred), os.path.getsize(os.path.join(HERE, "msra_sample.json")))

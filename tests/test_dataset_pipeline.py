@@ -3,7 +3,6 @@
 Golden fixtures (tests/golden/make_msra_sample_golden.py, make_variables_index_golden.py): the reference's own featurisation
 of its MSRA test split, recovered from the tokens / label_ids inside `data/msra/bilstm_crf_predict.pkl`; its
 `data_params.pkl`; the `variables.index` tables of its four serving checkpoints."""
-import hashlib
 import json
 import os
 import pickle
@@ -29,8 +28,8 @@ def _sample_dir(tmp_path):
     return str(tmp_path / "raw")
 
 
-def _prepare(tmp_path):
-    tok = TokenizerAdapter(SAMPLE["giga_vocab_subset"])
+def _prepare(tmp_path, vocab=None):
+    tok = TokenizerAdapter(SAMPLE["giga_vocab_subset"] if vocab is None else vocab)
     proc = bp.get_instance(TokenizerGiga, preprocess.MSRA_MAX_SEQ_LEN, preprocess.MSRA_TAG2IDX, tok)
     src, out = _sample_dir(tmp_path), str(tmp_path / "out")
     emb = np.random.default_rng(0).normal(size=(len(tok.vocab2idx), 50)).astype(np.float32)
@@ -57,6 +56,19 @@ def test_featurisation_equals_the_references_own_records(tmp_path):
     assert b["labels"][0][:5] == [{v: k for k, v in preprocess.MSRA_TAG2IDX.items()}[i] for i in SAMPLE["label_ids"][0][:5]]
 
 
+def test_out_of_vocabulary_characters_become_unk_in_the_references_records(tmp_path):
+    """The sample with every tenth vocabulary character removed: exactly the positions where the reference's record holds
+    a removed character become [UNK] (with the [UNK] id), everything else and every label_id stays the reference's."""
+    dropped = set(SAMPLE["giga_vocab_subset"][::10])
+    out, tok = _prepare(tmp_path, [c for c in SAMPLE["giga_vocab_subset"] if c not in dropped])
+    b = records.RecordFile(os.path.join(out, "giga_predict.nerrec")).batch(slice(0, 24))
+    want = [["[UNK]" if t in dropped else t for t in row] for row in SAMPLE["tokens"]]
+    assert b["tokens"] == want and sum(row.count("[UNK]") for row in want) > 24
+    assert b["label_ids"].tolist() == SAMPLE["label_ids"]
+    unk = b["token_ids"] == tok.vocab2idx["[UNK]"]
+    assert unk.tolist() == [[t == "[UNK]" for t in row] for row in want]
+
+
 def test_data_params_match_the_shipped_pickle(tmp_path):
     out, _ = _prepare(tmp_path)
     dp = pickle.load(open(os.path.join(out, "giga_data_params.pkl"), "rb"))
@@ -66,22 +78,6 @@ def test_data_params_match_the_shipped_pickle(tmp_path):
     assert dp["n_sample"] == 16 and dp["embedding"].shape[1] == 50
     ds = records.NerDataset(out, batch_size=5, epoch_size=3, model_name="bilstm_crf")
     assert ds.params["step_per_epoch"] == 3 and ds.params["num_train_steps"] == 9              # dataset.py:62-63
-
-
-@pytest.mark.skipif(not os.path.exists(os.path.join(os.path.dirname(GOLD), "..", "datasets", "msra", "giga_predict.nerrec")),
-                    reason="datasets/msra not generated (python -m chinesener_b200.data.preprocess ...)")
-def test_full_test_split_digest_matches_the_reference_pickle():
-    rec = records.RecordFile(os.path.join(os.path.dirname(GOLD), "..", "datasets", "msra", "giga_predict.nerrec"))
-    assert rec.n == SAMPLE["n_test"]
-    b = rec.batch(slice(0, rec.n))
-    h = hashlib.sha256()
-    for row in b["tokens"]:
-        h.update("\x1f".join(row).encode("utf-8") + b"\n")
-    assert h.hexdigest() == SAMPLE["tokens_sha256"]
-    h = hashlib.sha256()
-    for row in b["label_ids"].numpy():
-        h.update(bytes(int(x) for x in row))
-    assert h.hexdigest() == SAMPLE["label_ids_sha256"]
 
 
 def test_record_file_round_trip_with_optional_features(tmp_path):
@@ -180,7 +176,7 @@ def test_npz_checkpoint_keeps_adam_slots_and_global_step(tmp_path):
     assert float(fs3.slot_dict()["crf_layer/transitions"][0].abs().sum()) == 0.0
 
 
-def test_tf_bundle_index_reader_on_the_references_serving_checkpoints():
+def test_tf_bundle_index_reader_on_the_references_serving_checkpoints(tmp_path):
     gold = json.load(open(os.path.join(GOLD, "variables_index.json")))
     for model, g in gold.items():
         header, entries = tf_checkpoint.read_bundle_index(os.path.join(GOLD, "variables_index", model + ".index"), verify=True)
@@ -192,11 +188,12 @@ def test_tf_bundle_index_reader_on_the_references_serving_checkpoints():
     assert len(e) == 207 and sum(v["size"] for v in e.values()) == 412755392                 # BASELINE.md §1
     assert e["bilstm_layer/bidirectional_rnn/fw/multi_rnn_cell/cell_0/lstm_cell/kernel"]["shape"] == [896, 512]
     assert e["global_step"]["dtype"] == tf_checkpoint.DT_INT64 and e["global_step"]["shape"] == []
-    with pytest.raises(ValueError):                                                    # the data file is an LFS pointer upstream
-        open("/tmp/_ner_lfs.data-00000-of-00001", "wb").write(b"version https://git-lfs.github.com/spec/v1\n")
-        import shutil
-        shutil.copyfile(os.path.join(GOLD, "variables_index", "bilstm_crf.index"), "/tmp/_ner_lfs.index")
-        tf_checkpoint.load_tf_checkpoint("/tmp/_ner_lfs")
+    import shutil
+    prefix = str(tmp_path / "lfs")                                                     # the data file is an LFS pointer upstream
+    open(prefix + ".data-00000-of-00001", "wb").write(b"version https://git-lfs.github.com/spec/v1\n")
+    shutil.copyfile(os.path.join(GOLD, "variables_index", "bilstm_crf.index"), prefix + ".index")
+    with pytest.raises(ValueError):
+        tf_checkpoint.load_tf_checkpoint(prefix)
 
 
 def test_tf_bundle_write_read_round_trip(tmp_path):
