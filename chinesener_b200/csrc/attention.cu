@@ -227,6 +227,9 @@ extern "C" int ner_bert_attention(const void* qkv_bf16, const int32_t* mask, voi
       if (rc != NER_ERR_UNSUPPORTED) return rc;
     }
   }
+  // the K/V staging issues 16-byte cp.async copies (row stride 3*NH*64 bf16 keeps every row 16-byte aligned if the base is)
+  if ((reinterpret_cast<uintptr_t>(qkv_bf16) & 15) != 0 || (reinterpret_cast<uintptr_t>(ctx_bf16) & 15) != 0)
+    return NER_ERR_INVALID_ARG;
   const int Lp = (L + KB - 1) / KB * KB;
   const size_t smem = (size_t)2 * Lp * PITCH * 2 + (size_t)Lp * 4;
   if (smem > 227 * 1024) return NER_ERR_UNSUPPORTED;  // L <= ~780

@@ -319,6 +319,10 @@ static int attention_bwd_launch(const void* qkv_bf16, const int32_t* mask, const
   if (B == 0) return NER_OK;
   if (!qkv_bf16 || (!mask && !cu_seqlens) || !ctx_bf16 || !dctx_bf16 || !dqkv_bf16) return NER_ERR_INVALID_ARG;
   if (head_dim != D) return NER_ERR_UNSUPPORTED;
+  // Q/K/V and dO are staged with 16-byte cp.async copies, O is read and d_qkv written 4 bytes at a time
+  if ((reinterpret_cast<uintptr_t>(qkv_bf16) & 15) != 0 || (reinterpret_cast<uintptr_t>(dctx_bf16) & 15) != 0 ||
+      (reinterpret_cast<uintptr_t>(ctx_bf16) & 15) != 0 || (reinterpret_cast<uintptr_t>(dqkv_bf16) & 3) != 0)
+    return NER_ERR_INVALID_ARG;
   const int Lp = (L + 63) / 64 * 64;
   const size_t smem = (size_t)4 * Lp * PITCH * 2 + (size_t)4 * Lp * 4;
   if (smem > 227 * 1024) return NER_ERR_UNSUPPORTED;  // L <= ~380
